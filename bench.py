@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- edges/sec of the RGCN hot path on a PPI-shaped batch (BASELINE.json configs[1]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path over one batch: graph_num_layers = 3 x sparse_rgcn_layer
@@ -25,6 +25,10 @@ own counter (models/sparse_graph_model.py:285,310: sum of E_l per batch, counted
   sharded      (N > 1 only) BASELINE config 5 as ONE graph node-range sharded over the N GPUs through the library's own
                path (rgnn_halo_plan_create / rgnn_halo_exchange: peer-memory pull over NVLink, no NCCL on the data path):
                ms per layer, the exchange kernel alone, halo bytes, parity against the reference-generated fixture.
+  --dump-outputs DIR  after the timed steps, write what the last timed step computed (the final node states a caller of
+               the 3-layer stack receives) as DIR/node_states.npy (float32; node_states_rank<r>.npy on ranks > 0).  The
+               inputs are seeded, so runs with the same arguments can be compared output for output.  With --impl
+               reference, when a timed step is one of the three layers, one extra untimed 3-layer forward is dumped.
 Multi-GPU headline: weak scaling, every rank owns its own batch (graphs are independent units: no collective on the
 data path); value = edges of all ranks / max-over-ranks time.  The sharded block is the strong-scaling companion.
 """
@@ -59,6 +63,18 @@ def algorithmic_bytes_per_layer(V, M, L, D):
     """SURVEY.md 8(d): one gathered source row + (src,tgt) pair + in-degree scale per message, every node row
     read once and written once, the L weight matrices."""
     return M * (4 * D + 8 + 4) + V * 8 * D + L * D * D * 4
+
+
+def dump_outputs(args, rank, arrays):
+    """--dump-outputs: {name: array} -> DIR/<name>.npy (float32 / float64), a rank suffix on ranks > 0."""
+    import numpy as np
+    if not args.dump_outputs:
+        return
+    os.makedirs(args.dump_outputs, exist_ok=True)
+    for name, arr in arrays.items():
+        arr = np.asarray(arr)
+        assert arr.dtype in (np.float32, np.float64), (name, arr.dtype)
+        np.save(os.path.join(args.dump_outputs, name + ("_rank%d" % rank if rank else "") + ".npy"), arr)
 
 
 def make_inputs(seed):
@@ -165,8 +181,11 @@ def run_reference(args, rank, world):
         ref_torch.rgcn_stack(h, adj, cnt, step_ws)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        ref_torch.rgcn_stack(h, adj, cnt, step_ws)
+        out = ref_torch.rgcn_stack(h, adj, cnt, step_ws)
     dt = time.perf_counter() - t0
+    if layers_per_step < NUM_LAYERS:              # a timed step was one layer: the dump is the full stack's output (untimed)
+        out = ref_torch.rgcn_stack(h, adj, cnt, ws)
+    dump_outputs(args, rank, {"node_states": out.numpy()})
     ms = dt / args.steps * 1e3
     value = batch.num_edges / (dt / args.steps * NUM_LAYERS / layers_per_step)
     sample = "%d steps, each %d of the 3 RGCN layers over the full batch (%d edges); rate = edges / 3-layer time" % (
@@ -503,6 +522,7 @@ def run_ours(args, rank, world, local_rank):
     if sampler:
         sampler.start()
     total_ms, per_step = timed_steps(graph.replay, args.steps, args.warmup)
+    dump_outputs(args, rank, {"node_states": out_graph.cpu().numpy()})     # the replayed graph's output buffer: last timed step
     # roofline leg: ONE layer (transform GEMM + edge-stage segment kernel) as its own CUDA graph, same cold-L2
     # protocol -- the kernels' device time without host launch latency between them
     def one_layer():
@@ -762,7 +782,11 @@ def main():
     ap.add_argument("--skip-e2e", action="store_true", help="profiling runs: leave out the host-buffer leg")
     ap.add_argument("--skip-configs", action="store_true", help="leave out the lines for BASELINE configs 3-5")
     ap.add_argument("--skip-sharded", action="store_true", help="N > 1: leave out the node-range-sharded config-5 block")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's output (final node states) as DIR/node_states.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -171,22 +171,6 @@ def test_qm9_structure_archive_reproduces_the_full_validation_batch():
         assert r_struct["graph"] == r_real["graph"] and len(r_struct["node_features"]) == len(r_real["node_features"])
 
 
-def test_qm9_full_validation_set_counts_when_the_reference_data_is_present():
-    """SURVEY.md 8d config 3: 10,000 graphs, V = 180,560, M = 373,466 (L=4) / 554,026 (L=5).  Only runs where
-    /root/reference exists (the build container)."""
-    import os
-    import pytest
-    from tf_gnn_samples_b200 import batching
-    path = "/root/reference/data/qm9/valid.jsonl.gz"
-    if not os.path.exists(path):
-        pytest.skip("reference data not present")
-    recs = batching.load_qm9_jsonl(path)
-    b5, _, _ = batching.qm9_batch(recs)
-    b4, _, _ = batching.qm9_batch(recs, add_self_loop_edges=False)
-    assert (b5.num_graphs, b5.num_nodes, b5.num_edges, len(b5.adjacency_lists)) == (10000, 180560, 554026, 5)
-    assert (b4.num_nodes, b4.num_edges, len(b4.adjacency_lists)) == (180560, 373466, 4)
-
-
 def test_ppi_fold_loader_follows_the_reference(tmp_path):
     """tasks/ppi_task.py:68-160 on a tiny data set written in the dgl ppi.zip layout: two graphs interleaved in node-id
     ranges [0, 4) and [4, 7), links in arbitrary order."""

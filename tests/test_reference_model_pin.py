@@ -10,8 +10,10 @@ is committed as tests/golden/ref_model_<case>.npz and compared here:
 * everywhere: snapshot -> load_reference_checkpoint -> sort_variables -> oracle whole model on batching.py's feed == the
   reference's outputs (1e-12); snapshot -> SparseGraphModel.load_reference_weights -> every parameter lands where the
   oracle reads it; parameter counts equal the reference's;
-* where /root/reference exists: the same against a fresh run (the fixtures are current), default_params of every model
-  class, and README.md:29's 699257 parameters counted by the reference's own loop."""
+* against runs of the reference recorded in tests/golden/ref_records.json (tests/golden/ref_records.py models): the
+  fixtures are current, default_params of every model class, README.md:29's 699257 parameters counted by the reference's
+  own loop, the export direction (the reference's scaffold fed with a package model's values, its restore() of a snapshot
+  written here) and the train step."""
 import importlib
 import json
 import os
@@ -27,9 +29,9 @@ for p in (HERE, os.path.join(HERE, "golden")):
 
 import batcher_cases as BC      # noqa: E402
 import model_cases as MC        # noqa: E402
+import ref_records              # noqa: E402
 
 checkpoint = importlib.import_module("tf_gnn_samples_b200.checkpoint")
-have_reference = pytest.mark.skipif(not os.path.isdir("/root/reference/models"), reason="the reference checkout is not on this box")
 ALL = sorted(MC.CASES)
 
 
@@ -139,52 +141,58 @@ def test_default_params_of_the_snapshots_are_the_packages():
         assert extra <= {"max_epochs", "patience", "lr_for_num_graphs_per_batch"}, name
 
 
-# ---- against a fresh run of the reference (this container) ----
-@have_reference
+# ---- against a fresh run of the reference (recorded) ----
 @pytest.mark.parametrize("name", ALL)
-def test_fixture_equals_the_reference_scaffold_run_here(name):
+def test_fixture_equals_the_reference_scaffold_run_here(name, ppi_dir):
+    """The committed fixture equals a later, recorded run of the reference's scaffold (digests of the final node states and
+    every variable, parameter count, metrics); the oracle on batching.py's feed reproduces the fixture."""
     case = MC.CASES[name]
     z, snap = fixture(name)
-    r = MC.run_reference(case, np.float64)
-    assert np.array_equal(r["final"], z["final"]) and r["num_parameters"] == int(z["num_parameters"])
+    r = ref_records.load()["models"]["runs"][name]
+    assert ref_records.sha(z["final"]) == r["final"] and r["num_parameters"] == int(z["num_parameters"])
     assert sorted(r["variables"]) == list(z["variable_names"])
     for k, v in r["variables"].items():
-        assert np.array_equal(np.asarray(v, np.float64), np.asarray(snap.weights[k], np.float64)), k
-    check_metrics({k: float(v) for k, v in r["metrics"].items()}, json.loads(str(z["metrics"])), name)
-    o = MC.run_oracle(case, r["feed"], r["variables"], r["params"], r["task_params"], r["num_edge_types"])
-    assert rel(o["final"], r["final"]) <= 1e-12
+        assert ref_records.sha(np.asarray(snap.weights[k])) == v, k
+    check_metrics(r["metrics"], json.loads(str(z["metrics"])), name)
+    feed, L = repo_feed(case, snap.task_params, ppi_dir)          # bit-identical to the reference's feed (batcher pin)
+    o = MC.run_oracle(case, feed, snap.weights, snap.model_params, snap.task_params, L)
+    assert rel(o["final"], z["final"]) <= 1e-12
 
 
-@have_reference
 def test_readme_parameter_count_by_the_references_own_loop():
     """README.md:29 'Model has 699257 parameters' (RGCN on PPI: 50 features, 121 labels, 3 edge types, hidden 256, 3 layers),
     counted by sparse_graph_model.py:153-157 over the variables the reference's scaffold creates -- and by the package."""
     scaffold = importlib.import_module("tf_gnn_samples_b200.scaffold")
-    case = dict(kind="rgcn", task="ppi", model_params={"hidden_size": 256, "graph_num_layers": 3}, task_params={}, budget=10 ** 6)
-    r = MC.run_reference(case, np.float32, ppi_kw=dict(feature_dim=50, num_labels=121))
-    assert r["num_parameters"] == 699257
+    assert ref_records.load()["models"]["readme_num_parameters"] == 699257
     assert scaffold.RGCNPPIModel(device="cpu").num_parameters() == 699257
-    assert scaffold.SparseGraphModel("rgcn", "ppi", 3, 50, params=case["model_params"], device="cpu").num_parameters() == 699257
+    params = MC.README_RGCN_PPI["model_params"]
+    assert scaffold.SparseGraphModel("rgcn", "ppi", 3, 50, params=params, device="cpu").num_parameters() == 699257
 
 
-@have_reference
 def test_default_params_equal_the_reference_classes():
-    import tf1_shim
     scaffold = importlib.import_module("tf_gnn_samples_b200.scaffold")
-    with tf1_shim.installed():
-        tf1_shim.import_reference_task("sparse_graph_task")
-        import models
-        for kind, cls_name in MC.MODEL_CLASSES.items():
-            ref = getattr(models, cls_name).default_params()
-            mine = scaffold.model_default_params(kind)
-            for k, v in mine.items():
-                assert ref[k] == v, (kind, k, ref[k], v)
-            assert set(ref) - set(mine) <= {"max_epochs", "patience", "lr_for_num_graphs_per_batch"}, (kind, set(ref) - set(mine))
+    recorded = ref_records.load()["models"]["default_params"]
+    assert sorted(recorded) == sorted(MC.MODEL_CLASSES)
+    for kind, ref in recorded.items():
+        mine = scaffold.model_default_params(kind)
+        for k, v in mine.items():
+            assert ref[k] == ref_records.jsonable(v), (kind, k, ref[k], v)
+        assert set(ref) - set(mine) <= {"max_epochs", "patience", "lr_for_num_graphs_per_batch"}, (kind, set(ref) - set(mine))
 
 
 # ---- the export direction: a model of THIS package handed to the reference ----
+# The reference's side of these tests -- its scaffold fed with the exported values, its restore() of a snapshot written here, its
+# train step on prescribed gradients -- is recorded by tests/golden/ref_records.py (models) from the same package-side set-up.
 EXPORT_CASES = ["rgcn_ppi_scaffold", "film_ppi_scaffold", "rgin_ppi_scaffold", "ggnn_ppi_hidden_is_feature_size",
                 "rgcn_qm9", "ggnn_qm9", "rgat_qm9", "edge_mlp_qm9", "rgdcn_qm9"]
+RESTORE_CASES = ["rgin_ppi_scaffold", "edge_mlp_qm9", "ggnn_qm9"]
+OPTIMIZERS = ["SGD", "RMSProp", "Adam"]
+TASK_DEFAULTS = {"qm9": {"add_self_loop_edges": True, "tie_fwd_bkwd_edges": True, "task_ids": [0]},
+                 "ppi": {"add_self_loop_edges": True, "tie_fwd_bkwd_edges": False}}
+
+
+def recorded(section):
+    return ref_records.load()["models"][section]
 
 
 def _package_model(case, feed, L, seed):
@@ -211,83 +219,84 @@ def to_numpy(obj):
     return obj.detach().cpu().numpy()
 
 
-@have_reference
+def export_setup(name, ppi_dir):
+    """The seeded package model of an export case, its feed, and to_reference_weights() without the graph counter."""
+    case = MC.CASES[name]
+    feed, L = repo_feed(case, dict(TASK_DEFAULTS[case["task"]], **case["task_params"]), ppi_dir)
+    model, task_params = _package_model(case, feed, L, seed=5)
+    named = model.to_reference_weights()
+    counter = named.pop("total_num_graphs:0")
+    assert counter.dtype == np.int64 and counter.shape == ()
+    return case, feed, L, model, task_params, named
+
+
 @pytest.mark.parametrize("name", EXPORT_CASES)
 def test_exported_variables_drive_the_reference_scaffold(name, ppi_dir):
     """SparseGraphModel.to_reference_weights() names every variable the reference's scaffold creates (and nothing else); fed
     with those values the reference's own forward equals the oracle run on the model's weight dictionaries directly."""
     from oracle import ref_model
-    from tf1_shim import variables as TV
-    case = MC.CASES[name]
-    task_defaults = {"qm9": {"add_self_loop_edges": True, "tie_fwd_bkwd_edges": True, "task_ids": [0]},
-                     "ppi": {"add_self_loop_edges": True, "tie_fwd_bkwd_edges": False}}[case["task"]]
-    feed, L = repo_feed(case, dict(task_defaults, **case["task_params"]), ppi_dir)
-    model, task_params = _package_model(case, feed, L, seed=5)
-    named = model.to_reference_weights()
-    counter = named.pop("total_num_graphs:0")
-    assert counter.dtype == np.int64 and counter.shape == ()
-    provider = TV.provider_from(named)
-    r = MC.run_reference(case, np.float64, provider=provider)
-    assert provider.used == set(named), sorted(set(named) - provider.used)
-    assert set(r["variables"]) == set(named) | {"total_num_graphs:0"}
-    assert r["num_parameters"] == model.num_parameters()
+    case, feed, L, model, task_params, named = export_setup(name, ppi_dir)
+    ran = recorded("exported")[name]
+    assert ref_records.tree_digest(named) == ran["exported"]                   # the names and values the reference was fed
+    assert ref_records.tree_digest(sorted(named)) == ran["used"]               # it read every one of them ...
+    assert ref_records.tree_digest(sorted(set(named) | {"total_num_graphs:0"})) == ran["variables"]   # ... and created no other
+    assert ran["num_parameters"] == model.num_parameters()
     feats = np.asarray(feed["initial_node_features"], np.float32).astype(np.float64)
     adj = MC.adjacency_of(feed, L)
     indeg = np.asarray(feed["type_to_num_incoming_edges"], np.float32).astype(np.float64)
     final = ref_model.node_representations(model.kind, feats, adj, indeg, model.params, to_numpy(model.projection), to_numpy(model.layers))
-    assert rel(final, r["final"]) <= 1e-12
+    assert ref_records.summary_err(final, ran["final"]) <= 1e-12
     if case["task"] == "ppi":
         head = to_numpy(model.head)
         want = ref_model.ppi_metrics(final @ head["kernel"].astype(np.float64) + head["bias"], feed["target_labels"])
     else:
         outs = ref_model.qm9_outputs(final, feats, feed["graph_nodes_list"], int(feed["num_graphs"]), to_numpy(model.head))
         want = ref_model.qm9_metrics(outs, np.asarray(feed["target_values"]).astype(np.float32), task_params["task_ids"])
-    check_metrics(want, {k: float(v) for k, v in r["metrics"].items()}, name)
+    check_metrics(want, ran["metrics"], name)
 
 
-@have_reference
-@pytest.mark.parametrize("name", ["rgin_ppi_scaffold", "edge_mlp_qm9", "ggnn_qm9"])
-def test_the_references_restore_accepts_a_snapshot_written_here(name, ppi_dir, tmp_path, capsys):
-    """utils/model_utils.py:58-77 restore(): class names resolve, the task restores from the metadata, the model builds, and
-    load_weights finds a saved value for EVERY variable and uses EVERY saved value (it prints a line otherwise)."""
-    import tf1_shim
+def restore_setup(name, ppi_dir, directory):
+    """A seeded package model of a restore case, saved as a reference snapshot under ``directory``."""
     case = MC.CASES[name]
-    task_defaults = {"qm9": {"add_self_loop_edges": True, "tie_fwd_bkwd_edges": True, "task_ids": [0]},
-                     "ppi": {"add_self_loop_edges": True, "tie_fwd_bkwd_edges": False}}[case["task"]]
-    task_params = dict(task_defaults, out_layer_dropout_keep_prob=1.0, **case["task_params"])
+    task_params = dict(TASK_DEFAULTS[case["task"]], out_layer_dropout_keep_prob=1.0, **case["task_params"])
     feed, L = repo_feed(case, task_params, ppi_dir)
     model, _ = _package_model(case, feed, L, seed=9)
     F = feed["initial_node_features"].shape[1]
     metadata = {"params": task_params, "num_edge_types": L}
     metadata.update({"annotation_size": F} if case["task"] == "qm9" else
                     {"initial_node_feature_size": F, "num_labels": feed["target_labels"].shape[1]})
-    path = str(tmp_path / "snapshot.pickle")
+    path = os.path.join(directory, "snapshot.pickle")
     model.save_reference_snapshot(path, task_params, metadata)
-    with tf1_shim.installed(dtype=np.float32) as session:
-        session.feeds = dict(feed, out_layer_dropout_keep_prob=1.0)
-        mu = tf1_shim.import_reference_model_utils()
-        restored = mu.restore(path, str(tmp_path), run_id="restored")
-        out = capsys.readouterr().out
-        assert "Loaded model from snapshot" in out
-        assert "Freshly initializing" not in out and "not used by model" not in out, out
-        assert type(restored).__name__ == MC.MODEL_CLASSES[case["kind"]] and restored.task.num_edge_types == L
-        want = model.to_reference_weights()
-        for k, v in session.variables.items():
-            assert np.array_equal(np.asarray(v, np.float64), np.asarray(want[k], np.float64)), k
+    return case, feed, L, model, path
+
+
+@pytest.mark.parametrize("name", RESTORE_CASES)
+def test_the_references_restore_accepts_a_snapshot_written_here(name, ppi_dir, tmp_path):
+    """utils/model_utils.py:58-77 restore(): class names resolve, the task restores from the metadata, the model builds, and
+    load_weights finds a saved value for EVERY variable and uses EVERY saved value (it prints a line otherwise)."""
+    import pickle
+    case, feed, L, model, path = restore_setup(name, ppi_dir, str(tmp_path))
+    ran = recorded("restored")[name]
+    with open(path, "rb") as f:
+        assert ref_records.tree_digest(pickle.load(f)) == ran["snapshot"]      # the file the reference restored
+    out = ran["printed"]
+    assert "Loaded model from snapshot" in out
+    assert "Freshly initializing" not in out and "not used by model" not in out, out
+    assert ran["model_class"] == MC.MODEL_CLASSES[case["kind"]] and ran["num_edge_types"] == L
+    want = model.to_reference_weights()
+    assert sorted(ran["variables"]) == sorted(want)
+    for k, v in ran["variables"].items():
+        assert ref_records.sha(np.asarray(want[k], np.float64)) == v, k
 
 
 # ---- the train step (sparse_graph_model.py:226-260) ----
-@have_reference
-@pytest.mark.parametrize("optimizer", ["SGD", "RMSProp", "Adam"])
-def test_train_step_construction_and_per_tensor_clipping(optimizer, ppi_dir):
-    """__make_train_step run by the reference with PRESCRIBED gradients: which optimizer it builds with which hyper-parameters,
-    that the differentiated quantity is task_metrics['loss'], and that every gradient is clipped BY ITS OWN norm (tf.clip_by_norm,
-    not a global norm), None gradients passing through -- against scaffold.make_optimizer / clip_gradients_ on the same numbers."""
-    import torch
-    scaffold = importlib.import_module("tf_gnn_samples_b200.scaffold")
-    tfo = importlib.import_module("tf_gnn_samples_b200.tf_optimizers")
+def train_step_case(optimizer):
     hp = {"optimizer": optimizer, "learning_rate": 0.003, "learning_rate_decay": 0.9, "momentum": 0.7, "clamp_gradient_norm": 0.5}
-    case = dict(MC.CASES["film_ppi_scaffold"], model_params=dict(MC.CASES["film_ppi_scaffold"]["model_params"], **hp))
+    return dict(MC.CASES["film_ppi_scaffold"], model_params=dict(MC.CASES["film_ppi_scaffold"]["model_params"], **hp))
+
+
+def gradient_prescriber():
+    """The gradient the train step receives for each variable, drawn in the order the variables are asked for."""
     rng = np.random.default_rng(8)
     prescribed = {}
 
@@ -297,8 +306,23 @@ def test_train_step_construction_and_per_tensor_clipping(optimizer, ppi_dir):
         else:                                                    # norms on both sides of the clamp
             prescribed[name] = rng.standard_normal(shape) * (0.5 / np.sqrt(max(1, int(np.prod(shape))))) * rng.choice([0.2, 3.0])
         return prescribed[name]
+    return gradient_hook, prescribed
 
-    r = MC.run_reference(case, np.float64, gradient_hook=gradient_hook)
+
+@pytest.mark.parametrize("optimizer", OPTIMIZERS)
+def test_train_step_construction_and_per_tensor_clipping(optimizer, ppi_dir):
+    """__make_train_step run by the reference with PRESCRIBED gradients: which optimizer it builds with which hyper-parameters,
+    that the differentiated quantity is task_metrics['loss'], and that every gradient is clipped BY ITS OWN norm (tf.clip_by_norm,
+    not a global norm), None gradients passing through -- against scaffold.make_optimizer / clip_gradients_ on the same numbers.
+    The reference's clipped gradients are recorded as the factor it scaled each prescribed gradient by."""
+    import torch
+    scaffold = importlib.import_module("tf_gnn_samples_b200.scaffold")
+    tfo = importlib.import_module("tf_gnn_samples_b200.tf_optimizers")
+    case = train_step_case(optimizer)
+    r = recorded("train_step")[optimizer]
+    gradient_hook, prescribed = gradient_prescriber()
+    for name, shape in r["gradient_order"]:                      # the order the reference asked for them
+        gradient_hook(name, tuple(shape))
     assert r["loss_is_task_loss"]
     (cls_name, kwargs), = r["optimizers"]
     feed, L = repo_feed(case, {"add_self_loop_edges": True, "tie_fwd_bkwd_edges": True}, ppi_dir)
@@ -324,7 +348,7 @@ def test_train_step_construction_and_per_tensor_clipping(optimizer, ppi_dir):
     pre = {n: None if p.grad is None else float(p.grad.norm()) for n, p in named.items()}
     assert min(v for v in pre.values() if v is not None) < 0.5 < max(v for v in pre.values() if v is not None)
     model.clip_gradients_()
-    applied = dict((n, g) for g, n in r["applied"])
+    applied = {n: None if s is None else s * prescribed[n] for n, s in r["applied_scale"].items()}
     assert set(applied) == set(named)
     for name, p in named.items():
         if prescribed[name] is None:
@@ -334,16 +358,18 @@ def test_train_step_construction_and_per_tensor_clipping(optimizer, ppi_dir):
             assert float(np.linalg.norm(applied[name])) <= 0.5 * (1 + 1e-12)
 
 
-@have_reference
-def test_learning_rate_normalised_per_graph_count(ppi_dir):
+def lr_case():
+    hp = {"optimizer": "RMSProp", "learning_rate": 0.003, "lr_for_num_graphs_per_batch": 30}
+    return dict(MC.CASES["rgcn_qm9"], model_params=dict(MC.CASES["rgcn_qm9"]["model_params"], **hp))
+
+
+def test_learning_rate_normalised_per_graph_count():
     """lr_for_num_graphs_per_batch = n (sparse_graph_model.py:230-238): the reference hands the optimizer
     learning_rate * num_graphs / n; set_learning_rate_ puts the same number into the torch optimizer before the step."""
     scaffold = importlib.import_module("tf_gnn_samples_b200.scaffold")
-    hp = {"optimizer": "RMSProp", "learning_rate": 0.003, "lr_for_num_graphs_per_batch": 30}
-    case = dict(MC.CASES["rgcn_qm9"], model_params=dict(MC.CASES["rgcn_qm9"]["model_params"], **hp))
-    r = MC.run_reference(case, np.float32)
+    r = recorded("lr_per_graph_count")
     (cls_name, kwargs), = r["optimizers"]
-    G = int(r["feed"]["num_graphs"])
+    G = r["num_graphs"]
     assert cls_name == "RMSPropOptimizer" and G not in (0, 30)
     model = scaffold.SparseGraphModel("rgcn", "qm9", r["num_edge_types"], 15, params=r["params"], task_ids=(0, 4), device="cpu")
     opt = model.make_optimizer()

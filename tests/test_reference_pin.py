@@ -4,9 +4,10 @@
   test_oracle_matches_reference_fixture      oracle float64 == reference-through-shim float64 to 1e-12 (small cases: every
                                              element; BASELINE configs 2-5: committed rows + projection + column sums), and
                                              the oracle's float32 mode tracks the reference's float32 arithmetic;
-  test_reference_code_reproduces_fixtures    (only where /root/reference exists, i.e. in the build container) re-executes the
-                                             reference through the shim and checks the committed files and the oracle against
-                                             it element by element -- so the fixtures cannot drift from the reference;
+  test_reference_code_reproduces_fixtures    the reference re-executed through the shim (recorded in tests/golden/ref_records.json
+                                             by tests/golden/ref_records.py layer_fixtures: the variables it created and a seeded
+                                             summary of its float64 output) against the committed files and the oracle -- so
+                                             the fixtures cannot drift from the reference;
   test_variable_names_round_trip             the variables the reference creates, sorted by checkpoint.sort_variables, feed the
                                              oracle and reproduce the same output (pins the TF-name mapping both ways);
   test_engine_matches_reference_fixture      -m gpu: the CUDA engine through the C ABI against the same fixtures at 1e-4, and
@@ -25,14 +26,15 @@ sys.path.insert(0, os.path.join(HERE, "golden"))
 sys.path.insert(0, HERE)
 
 import ref_cases as RC                       # noqa: E402
+import ref_records                           # noqa: E402
 from oracle import ref_layers as R           # noqa: E402
 from helpers import assert_parity            # noqa: E402
 
-HAVE_REFERENCE = os.path.isdir("/root/reference/gnns")
 SMALL = [n for n, c in RC.CASES.items() if not c.get("big")]
 BIG = [n for n, c in RC.CASES.items() if c.get("big")]
 # the heavy float64 oracle passes (QM9-10k x 4 timesteps, 1M-edge FiLM) take tens of seconds each: CPU suite runs them once
 BIG_CPU = ["config2_rgcn_ppi", "config4_rgat_ppi", "config5_film_random", "config3_ggnn_qm9"]
+REEXECUTED = SMALL + ["config2_rgcn_ppi", "config4_rgat_ppi"]
 
 
 def load(name):
@@ -78,24 +80,19 @@ def test_oracle_matches_reference_fixture_baseline_configs(name):
     assert max(err_rows, err_proj, err_col) <= 1e-12, (err_rows, err_proj, err_col)
 
 
-@pytest.mark.skipif(not HAVE_REFERENCE, reason="/root/reference is only present in the build container")
-@pytest.mark.parametrize("name", SMALL + ["config2_rgcn_ppi", "config4_rgat_ppi"])
+@pytest.mark.parametrize("name", REEXECUTED)
 def test_reference_code_reproduces_fixtures(name):
-    import warnings
-    import make_ref_fixtures as MRF
     case, z = RC.CASES[name], load(name)
+    ran = ref_records.load()["layer_fixtures"][name]
     h, adj, indeg = case["graph"]()
     w = case["weights"]()
-    with warnings.catch_warnings():
-        warnings.simplefilter("ignore")       # the reference's docstrings hold '\e' escapes (SyntaxWarning on 3.12)
-        out64, created = MRF.run_reference(case, h, adj, indeg, w, np.float64)
-    assert sorted(created) == [str(s) for s in z["variable_names"]]
+    assert ran["created"] == [str(s) for s in z["variable_names"]]
     o64 = oracle_run(case, h, adj, indeg, w, np.float64)
-    assert R.max_norm_rel_err(o64, out64) <= 1e-12              # every element, also for the BASELINE-sized cases
-    if case.get("big"):
-        assert max(RC.compare_with_summary(out64, z, name)) <= 1e-13
+    assert ref_records.summary_err(o64, ran["out"]) <= 1e-12
+    if case.get("big"):                        # committed rows, projection, column sums = those of the re-executed run
+        assert {k: ref_records.sha(z[k]) for k in ran["fixture_summary"]} == ran["fixture_summary"]
     else:
-        np.testing.assert_allclose(out64, z["out"], rtol=0, atol=1e-13)
+        assert ref_records.summary_err(z["out"], ran["out"]) <= 1e-13
 
 
 @pytest.mark.parametrize("name", SMALL)

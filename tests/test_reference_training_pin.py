@@ -6,16 +6,16 @@ PPI fold, train + valid), its batcher makes the minibatches, ``sess.run`` is SCR
 metric dictionary per batch and records the feed_dict the loop assembled), the clock is a counter.  training.train gets the
 same data through batching.py, a stub model producing the same scripted metrics and the same clock -- and must write the
 same log, line for line: epoch headers, Train / Valid lines with loss, MAE / error ratios or micro-F1, graphs / nodes /
-edges per second, save-best lines, early stopping after ``patience`` epochs, the final summary.  Needs /root/reference."""
+edges per second, save-best lines, early stopping after ``patience`` epochs, the final summary.  The reference's log and the
+minibatches its loop fed are recorded in tests/golden/ref_records.json (tests/golden/ref_records.py training), with the
+data directory written as <DIR>."""
 import gzip
 import importlib
 import json
 import os
 import sys
-import types
 
 import numpy as np
-import pytest
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 for p in (HERE, os.path.join(HERE, "golden")):
@@ -23,8 +23,8 @@ for p in (HERE, os.path.join(HERE, "golden")):
         sys.path.insert(0, p)
 
 import batcher_cases as BC      # noqa: E402
+import ref_records              # noqa: E402
 
-pytestmark = pytest.mark.skipif(not os.path.isdir("/root/reference/models"), reason="the reference checkout is not on this box")
 batching = importlib.import_module("tf_gnn_samples_b200.batching")
 training = importlib.import_module("tf_gnn_samples_b200.training")
 
@@ -63,64 +63,6 @@ def write_qm9_folds(d):
             for r in part:
                 f.write(json.dumps(r) + "\n")
     return recs[:150], recs[150:]
-
-
-def run_reference_loop(task_name, data_dir, task_params, model_params, max_nodes=MAX_NODES, test_path=None):
-    import tf1_shim
-    calls = []
-    with tf1_shim.installed(dtype=np.float32) as session:
-        from dpu_utils.utils import RichPath
-        sgt = tf1_shim.import_reference_task("sparse_graph_task")
-        mod = tf1_shim.import_reference_task(task_name + "_task")
-        cls = mod.QM9_Task if task_name == "qm9" else mod.PPI_Task
-        params = cls.default_params()
-        params.update(task_params)
-        task = cls(params)
-        task.load_data(RichPath.create(data_dir))
-        target = "target_values" if task_name == "qm9" else "target_labels"
-        names = ["initial_node_features", "type_to_num_incoming_edges", "graph_nodes_list", target, "out_layer_dropout_keep_prob"]
-        feed = BC._feeds_of(task, list(task._loaded_data[sgt.DataFold.VALIDATION]), sgt.DataFold.VALIDATION, names, max_nodes)[0]
-        session.feeds = feed                                       # only to BUILD the model; the loop's results are scripted
-        import models
-        import models.sparse_graph_model as sgm
-        mparams = models.GGNN_Model.default_params()
-        mparams.update(model_params)
-        model = models.GGNN_Model(mparams, task, "run", data_dir)
-        ph = model._Sparse_Graph_Model__placeholders
-        state = {"epoch": 1, "fold": None, "step": 0}
-
-        def hook(fetches, feed_dict):
-            if not isinstance(fetches, dict) or "task_metrics" not in fetches:       # save_model's variable fetch
-                return {k: v.value() for k, v in fetches.items()}
-            fold = "train" if "train_step" in fetches else "valid"
-            if state["epoch"] == 99:
-                fold = "test"
-            if fold != state["fold"]:
-                if fold == "train" and state["fold"] == "valid":
-                    state["epoch"] += 1
-                state["fold"], state["step"] = fold, 0
-            g = int(feed_dict[ph["num_graphs"]])
-            calls.append({"fold": fold, "epoch": state["epoch"], "num_graphs": g,
-                          "num_nodes": int(np.asarray(feed_dict[ph["initial_node_features"]]).shape[0]),
-                          "keep_prob_fed": ph["graph_layer_input_dropout_keep_prob"] in feed_dict,
-                          "first_feature_row": np.asarray(feed_dict[ph["initial_node_features"]])[0].astype(np.float32)})
-            out = {"task_metrics": scripted(task_name, fold, state["epoch"], state["step"], g, params.get("task_ids", [0]))}
-            state["step"] += 1
-            return out
-
-        session.run_hook = hook
-        sgm.time = types.SimpleNamespace(time=make_counter_clock())   # the module's clock; the source file is untouched
-        try:
-            model.train(quiet=True)
-            if test_path is not None:                            # Sparse_Graph_Model.test (:373-385) on a held-out file / fold
-                state.update(epoch=99, fold=None, step=0)
-                model.test(RichPath.create(test_path), quiet=True)
-        finally:
-            import time as real_time
-            sgm.time = real_time
-        with open(model.log_file) as f:
-            lines = f.read().splitlines()
-        return lines, calls, model.best_model_file, os.path.exists(model.best_model_file)
 
 
 class ScriptedModel:
@@ -179,29 +121,45 @@ def run_package_loop(task, train_samples, valid_samples, task_ids, best_model_fi
     return lines, model.calls, saves, res
 
 
+def write_qm9_data(d):
+    """150 training and 50 validation molecules, and a held-out file of 80 of them."""
+    train_recs, valid_recs = write_qm9_folds(d)
+    test_file = os.path.join(d, "heldout.jsonl.gz")
+    with gzip.open(test_file, "wt") as f:
+        for r in (train_recs + valid_recs)[40:120]:
+            f.write(json.dumps(r) + "\n")
+    return train_recs, valid_recs, test_file
+
+
+def write_ppi_data(d):
+    BC.write_ppi_dir(d, "train", seed=1, num_graphs=9)
+    BC.write_ppi_dir(d, "valid", seed=2, num_graphs=4)
+    BC.write_ppi_dir(d, "test", seed=3, num_graphs=3)
+
+
+def recorded_reference_loop(task, data_dir):
+    """The reference's log lines, the minibatches its loop fed and its best-model file, for data written to ``data_dir``."""
+    r = ref_records.load()["training"][task]
+    assert r["saved"]
+    return ([line.replace("<DIR>", data_dir) for line in r["lines"]], r["calls"],
+            os.path.join(data_dir, r["best_model_file"]))
+
+
 def compare(ref_lines, ref_calls, pkg_lines, pkg_calls):
     assert ref_lines[0].startswith("Model has ") and ref_lines[1:] == pkg_lines, "\n".join(
         "%s\n%s" % (a, b) for a, b in zip(ref_lines[1:], pkg_lines) if a != b)
     assert len(ref_calls) == len(pkg_calls)
     for a, b in zip(ref_calls, pkg_calls):                        # the same minibatches in the same (shuffled) order
         assert (a["fold"], a["epoch"], a["num_graphs"], a["num_nodes"]) == (b["fold"], b["epoch"], b["num_graphs"], b["num_nodes"])
-        assert np.array_equal(a["first_feature_row"], np.asarray(b["first_feature_row"], np.float32))
+        assert a["first_feature_row"] == ref_records.sha(np.asarray(b["first_feature_row"], np.float32))
         assert a["keep_prob_fed"] == (a["fold"] == "train")       # dropout keep-prob only fed while training (:277-279)
     assert {c["fold"] for c in ref_calls} == {"train", "valid", "test"}
 
 
 def test_qm9_epoch_loop_writes_the_references_log(tmp_path):
-    train_recs, valid_recs = write_qm9_folds(str(tmp_path))
+    train_recs, valid_recs, test_file = write_qm9_data(str(tmp_path))
     task_ids = [0, 4]
-    test_file = os.path.join(str(tmp_path), "heldout.jsonl.gz")
-    with gzip.open(test_file, "wt") as f:
-        for r in (train_recs + valid_recs)[40:120]:
-            f.write(json.dumps(r) + "\n")
-    ref_lines, ref_calls, best_file, saved = run_reference_loop(
-        "qm9", str(tmp_path), {"task_ids": task_ids},
-        {"hidden_size": 16, "graph_num_layers": 1, "max_nodes_in_batch": MAX_NODES, "patience": PATIENCE, "random_seed": SEED},
-        test_path=test_file)
-    assert saved
+    ref_lines, ref_calls, best_file = recorded_reference_loop("qm9", str(tmp_path))
     L = batching.qm9_num_edge_types(train_recs + valid_recs)
     samples = lambda recs: [batching.qm9_graph_to_sample(r, L) for r in recs]
     held_out = samples(batching.load_qm9_jsonl(test_file))
@@ -217,13 +175,8 @@ def test_qm9_epoch_loop_writes_the_references_log(tmp_path):
 
 def test_ppi_epoch_loop_writes_the_references_log(tmp_path):
     d = str(tmp_path)
-    BC.write_ppi_dir(d, "train", seed=1, num_graphs=9)
-    BC.write_ppi_dir(d, "valid", seed=2, num_graphs=4)
-    BC.write_ppi_dir(d, "test", seed=3, num_graphs=3)
-    ref_lines, ref_calls, best_file, saved = run_reference_loop(
-        "ppi", d, {}, {"hidden_size": 16, "graph_num_layers": 1, "max_nodes_in_batch": 120, "patience": PATIENCE, "random_seed": SEED},
-        max_nodes=120, test_path=d)
-    assert saved
+    write_ppi_data(d)
+    ref_lines, ref_calls, best_file = recorded_reference_loop("ppi", d)
     tr, _ = batching.load_ppi_fold(d, "train")
     va, _ = batching.load_ppi_fold(d, "valid")
     te, _ = batching.load_ppi_fold(d, "test")

@@ -1,7 +1,7 @@
 """utils/utils.py's name factories (get_activation, get_aggregation_function, get_gated_unit) and utils/model_utils.py's
 name_to_model_class: the names accepted, the exception types and messages raised -- the REFERENCE's functions (run under
-tests/tf1_shim) against the package's.  Needs /root/reference (skipped on the GPU box; the committed known-answer tests in
-test_parity_traps.py / test_abi_and_host.py cover the same names without it)."""
+tests/tf1_shim) against the package's.  What the reference returned or raised for every name is stored in
+tests/golden/ref_records.json (tests/golden/ref_records.py utils)."""
 import importlib
 import os
 import sys
@@ -10,10 +10,12 @@ import numpy as np
 import pytest
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-if HERE not in sys.path:
-    sys.path.insert(0, HERE)
+for _p in (HERE, os.path.join(HERE, "golden")):
+    if _p not in sys.path:
+        sys.path.insert(0, _p)
 
-pytestmark = pytest.mark.skipif(not os.path.isdir("/root/reference/utils"), reason="the reference checkout is not on this box")
+import ref_records                                           # noqa: E402
+
 mine = importlib.import_module("tf_gnn_samples_b200.utils")
 scaffold = importlib.import_module("tf_gnn_samples_b200.scaffold")
 
@@ -27,103 +29,86 @@ MODEL_NAMES = ["ggnn", "GGNN", "ggnn_model", "gnn_edge_mlp", "gnn-edge-mlp", "GN
                "rgat_model", "rgcn", "RGCN", "rgcn_model", "rgdcn", "rgdcn_model", "rgin", "RGIN", "rgin_model", "gcn", "gat", ""]
 
 
-def outcome(fn, *args):
-    try:
-        return ("ok", fn(*args))
-    except Exception as e:                                   # noqa: BLE001 -- the exception IS the behaviour under test
-        return (type(e).__name__, str(e))
+outcome = ref_records.outcome
 
 
 @pytest.fixture(scope="module")
 def reference():
-    import tf1_shim
-    with tf1_shim.installed(dtype=np.float64) as session:
-        import utils as ref_utils
-        mu = tf1_shim.import_reference_model_utils()
-        yield ref_utils, mu, session
+    return ref_records.load()["utils"]
 
 
 def test_activation_names_and_errors(reference):
-    ref_utils, _, session = reference
+    import math
     x = np.linspace(-3, 3, 25)
-    tf = session.tf
+    elu = lambda v: np.where(v > 0, v, np.expm1(np.minimum(v, 0)))                          # noqa: E731
     values = {mine.ACT_LINEAR: lambda v: v, mine.ACT_TANH: np.tanh, mine.ACT_RELU: lambda v: np.maximum(v, 0),
-              mine.ACT_LEAKY_RELU: lambda v: np.where(v > 0, v, 0.2 * v), mine.ACT_ELU: tf.nn.elu, mine.ACT_SELU: tf.nn.selu,
-              mine.ACT_GELU: lambda v: v * 0.5 * (1.0 + tf.erf(v / np.sqrt(2.0)))}
-    for name in ACTIVATION_NAMES:
-        ref, got = outcome(ref_utils.get_activation, name), outcome(mine.get_activation, name)
+              mine.ACT_LEAKY_RELU: lambda v: np.where(v > 0, v, 0.2 * v), mine.ACT_ELU: elu,
+              mine.ACT_SELU: lambda v: 1.0507009873554804934193349852946 * np.where(v > 0, v, 1.6732632423543772848170429916717 * np.expm1(np.minimum(v, 0))),
+              mine.ACT_GELU: lambda v: v * 0.5 * (1.0 + np.vectorize(math.erf)(v / np.sqrt(2.0)))}
+    assert len(reference["activation"]) == len(ACTIVATION_NAMES)
+    for name, ref in zip(ACTIVATION_NAMES, reference["activation"]):
+        got = outcome(mine.get_activation, name)
         if ref[0] != "ok":
             assert got == ref, (name, got, ref)               # same exception type, same message
             continue
         assert got[0] == "ok", (name, got)
-        fn = ref[1]
-        want = x if fn is None else fn(x)                    # None = no activation (rgcn.py:112 etc. guard on it)
+        want = np.array(ref[1])                              # the reference's function on x (None = no activation: x itself)
         assert np.allclose(values[got[1]](x), want, rtol=0, atol=1e-15), name
 
 
 def test_aggregation_names_and_errors(reference):
-    ref_utils, _, session = reference
-    tf = session.tf
-    codes = {mine.AGG_SUM: tf.unsorted_segment_sum, mine.AGG_MAX: tf.unsorted_segment_max, mine.AGG_MEAN: tf.unsorted_segment_mean,
-             mine.AGG_SQRT_N: tf.unsorted_segment_sqrt_n}
-    for name in AGGREGATION_NAMES:
-        ref, got = outcome(ref_utils.get_aggregation_function, name), outcome(mine.get_aggregation_function, name)
+    codes = {mine.AGG_SUM: "sum", mine.AGG_MAX: "max", mine.AGG_MEAN: "mean", mine.AGG_SQRT_N: "sqrt_n"}
+    assert len(reference["aggregation"]) == len(AGGREGATION_NAMES)
+    for name, ref in zip(AGGREGATION_NAMES, reference["aggregation"]):
+        got = outcome(mine.get_aggregation_function, name)
         if ref[0] != "ok":
             assert got == ref, (name, got, ref)
         else:
-            assert got[0] == "ok" and codes[got[1]] is ref[1], (name, got, ref)
+            assert got[0] == "ok" and codes[got[1]] == ref[1], (name, got, ref)
 
 
 def test_gated_unit_names_and_errors(reference):
-    ref_utils, _, _ = reference
-    for name in CELL_NAMES:
-        ref, got = outcome(ref_utils.get_gated_unit, 8, name, "tanh"), outcome(mine.get_gated_unit, 8, name, "tanh")
+    assert len(reference["gated_unit"]) == len(CELL_NAMES)
+    for name, ref in zip(CELL_NAMES, reference["gated_unit"]):
+        got = outcome(mine.get_gated_unit, 8, name, "tanh")
         if name.lower() == "lstm":                            # constructs in the reference, cannot be CALLED there (ggnn.py:92)
-            assert ref[0] == "ok" and got[0] == "NotImplementedError"
-            with pytest.raises(ValueError):
-                ref[1](np.zeros((2, 8)), [np.zeros((2, 8))])
+            assert ref[0] == "ok" and ref[2] == "ValueError" and got[0] == "NotImplementedError"
             continue
         if ref[0] != "ok":
             assert got == ref, (name, got, ref)
         else:
-            cell = {"_SimpleRNNCell": mine.CELL_RNN, "_GRUCell": mine.CELL_GRU}[type(ref[1]).__name__]
-            assert got == ("ok", (cell, mine.ACT_TANH)), (name, got)
-    assert outcome(mine.get_gated_unit, 8, "gru", "swish") == outcome(ref_utils.get_gated_unit, 8, "gru", "swish")
+            cell = {"_SimpleRNNCell": mine.CELL_RNN, "_GRUCell": mine.CELL_GRU}[ref[1]]
+            assert got == ["ok", (cell, mine.ACT_TANH)], (name, got)
+    assert outcome(mine.get_gated_unit, 8, "gru", "swish") == reference["gated_unit_gru_swish"]
 
 
 def test_model_names_resolve_like_name_to_model_class(reference):
-    _, mu, _ = reference
     import test_reference_model_pin as P
     kinds = {v: k for k, v in P.MC.MODEL_CLASSES.items()}
-    for name in MODEL_NAMES:
-        ref, got = outcome(mu.name_to_model_class, name), outcome(scaffold.model_default_params, name)
+    assert len(reference["model_names"]) == len(MODEL_NAMES)
+    for name, ref in zip(MODEL_NAMES, reference["model_names"]):
+        got = outcome(scaffold.model_default_params, name)
         if ref[0] != "ok":
             assert got == ref, (name, got, ref)
             continue
-        cls, extra = ref[1]
+        _, cls_name, want = ref
         assert got[0] == "ok", (name, got)
-        want = cls.default_params()
-        want.update(extra)
         for k, v in got[1].items():
-            assert want[k] == v, (name, k, want[k], v)
-        assert scaffold.resolve_model_name(name)[0] == kinds[cls.__name__], name
+            assert want[k] == ref_records.jsonable(v), (name, k, want[k], v)
+        assert scaffold.resolve_model_name(name)[0] == kinds[cls_name], name
 
 
 def test_layer_function_signatures_equal_the_references(reference):
     """gnns/__init__.py exports seven sparse_<x>_layer functions; the package's take the same positional / keyword parameters in
     the same order with the same defaults, plus keyword-only extras (weights=, plan=, ...) that the reference cannot know."""
     import inspect
-    import gnns as ref_gnns                                   # the reference's package (inside the fixture's installed() block)
     pkg = importlib.import_module("tf_gnn_samples_b200.gnns")
-    names = [n for n in dir(ref_gnns) if n.startswith("sparse_") and n.endswith("_layer")]
-    assert sorted(names) == ["sparse_ggnn_layer", "sparse_gnn_edge_mlp_layer", "sparse_gnn_film_layer", "sparse_rgat_layer",
-                             "sparse_rgcn_layer", "sparse_rgdcn_layer", "sparse_rgin_layer"]
-    for n in names:
-        ref = inspect.signature(getattr(ref_gnns, n)).parameters
+    signatures = reference["layer_signatures"]
+    assert sorted(signatures) == ["sparse_ggnn_layer", "sparse_gnn_edge_mlp_layer", "sparse_gnn_film_layer", "sparse_rgat_layer",
+                                  "sparse_rgcn_layer", "sparse_rgdcn_layer", "sparse_rgin_layer"]
+    for n, ref in signatures.items():
         got = inspect.signature(getattr(pkg, n)).parameters
         shared = [p for p in got.values() if p.kind != inspect.Parameter.KEYWORD_ONLY]
-        assert [p.name for p in shared] == list(ref), (n, [p.name for p in shared], list(ref))
-        for p in shared:
-            assert p.default == ref[p.name].default, (n, p.name, p.default, ref[p.name].default)
+        assert [[p.name, repr(p.default)] for p in shared] == ref, (n, [p.name for p in shared], ref)
         extras = [p.name for p in got.values() if p.kind == inspect.Parameter.KEYWORD_ONLY]
         assert "weights" in extras, (n, extras)
